@@ -18,6 +18,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, "/root/reference")
 
+torch.set_num_threads(10)      # fp32 reductions depend on it; tests/test_oracle_golden.py runs with the same count
 sp.dok_matrix._update = lambda self, d: [self.__setitem__(k, v) for k, v in d.items()]
 _m, _mp = types.ModuleType("matplotlib"), types.ModuleType("matplotlib.pyplot")
 _m.pyplot = _mp

@@ -327,16 +327,37 @@ def test_device_graph_builder_matches_host_builder():
     assert np.array_equal(a.seg_host, b.seg_host)
 
 
-REFERENCE = "/root/reference/FoodRec"
+# The parts of the reference's `FoodRec/` tree that model discovery touches: the lookup of its `get_model`
+# (FoodRec/utils/utils.py:27-40, `importlib` on `models.<name.lower()>`) and a `models` package holding modules of the
+# same names as the drop-ins, so the test also fails if the reference's own files won.
+_REFERENCE_LAYOUT = {
+    "utils/__init__.py": "",
+    "utils/utils.py": (
+        "import importlib\n"
+        "import importlib.util\n\n\n"
+        "def get_model(model_name):\n"
+        "    module_path = '.'.join(['models', model_name.lower()])\n"
+        "    if importlib.util.find_spec(module_path, __name__):\n"
+        "        model_module = importlib.import_module(module_path, __name__)\n"
+        "    return getattr(model_module, model_name)\n"),
+    "models/__init__.py": "",
+    **{f"models/{name.lower()}.py": f"class {name}:\n    pass\n"
+       for name in ("PRICAI_ModelX", "CIKM_Model", "LightGCN", "SCHGN", "BM3")},
+}
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="the reference checkout only exists in the build container")
-def test_unmodified_get_model_resolves_the_dropins():
-    """Zero-edit discovery (SURVEY.md 8b): with `dropin/` ahead of `FoodRec/` on sys.path the reference's own
-    `get_model` (FoodRec/utils/utils.py:27-40) returns the B200 classes for the four hot-path models and still finds
-    the reference's other models through the overlay's `__path__`."""
+def test_unmodified_get_model_resolves_the_dropins(tmp_path):
+    """Zero-edit discovery (SURVEY.md 8b): with `dropin/` ahead of `FoodRec/` on sys.path the reference's
+    `get_model` returns the B200 classes for the four hot-path models and still finds the reference's other models
+    through the overlay's `__path__`."""
     import subprocess
     import sys
+    REFERENCE = str(tmp_path / "FoodRec")
+    for rel, src in _REFERENCE_LAYOUT.items():
+        path = os.path.join(REFERENCE, rel)
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, "w") as f:
+            f.write(src)
     code = (
         "import sys, types\n"
         f"sys.path[:0] = [{os.path.join(ROOT, 'dropin')!r}, {REFERENCE!r}, {os.path.dirname(REFERENCE)!r}]\n"   # bm3.py imports `FoodRec.common...`

@@ -8,6 +8,18 @@ from conftest import load_golden
 from oracle import adjacency, knn, losses, propagation, ranking
 
 RTOL = 1e-5
+# The goldens were written with 10 torch intra-op threads.  Several compared values (SCHGN's attention-weight
+# gradients among them) are fp32 sums with heavy cancellation that move by up to 1e-4 relative with the number of
+# threads a reduction is split over, so the oracle runs with the same count on every host.
+GOLDEN_THREADS = 10
+
+
+@pytest.fixture(autouse=True)
+def golden_thread_count():
+    prev = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(prev)
 
 
 def close(a, b, rtol=RTOL, atol=1e-7):
