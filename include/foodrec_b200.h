@@ -391,6 +391,43 @@ int fr_sample_negatives(const int64_t *excl_ptr, const int32_t *excl_idx, const 
                         int32_t n_items, uint64_t seed, uint64_t step, int64_t *out_neg, int32_t *fail_count,
                         void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Evaluation metrics on the device (the host step after full-sort / by-user ranking: metrics.topk_metrics and
+ * metrics.by_user_metrics, FoodRec/utils/topk_evaluator.py:68-115, FoodRec/common/matrics.py:9-102,
+ * FoodRec/common/trainer.py:49-69,231-282).  Both write SUMS over users in fp64 (the caller divides); per-user values
+ * are optional.  Block partials are folded by the last block in a fixed order: bit-reproducible on a given device.
+ * `ws`: fr_eval_metrics_ws_bytes() bytes, 16-byte aligned, zeroed once; its ticket word is left zero, so the
+ * launches replay inside a CUDA graph.  One `ws` serves both entry points, one launch at a time.
+ *
+ * fr_topk_metrics: top [n, K] (int32, or int64 with idx64 != 0; K <= 64; entries < 0 are padding, never a hit) against
+ * the held-out positives pos_idx[pos_ptr[r] .. pos_ptr[r+1]) (sorted, unique per row), pos_len[r] = the length of the
+ * list as given (duplicates included: the host divides by it); cutoffs c_i in 1..K.  A repeated column counts as a hit
+ * each time.  disc / ideal [K] fp32: 1 / log2(rank + 1) and its running sum, computed by the caller with numpy's
+ * expressions (metrics._ndcg_tables).  Per user and cutoff c, with cum = hits in the first c columns:
+ *   recall = cum / pos_len, precision = cum / c (fp64); recall2 contributes cum (its mean = sum cum / sum pos_len);
+ *   ndcg = (fp32 running sum of disc over the hit columns) / ideal[min(c, pos_len) - 1] (fp32);
+ *   map = fp32( (sum over hit columns j < c of cum_j / (j + 1), fp64) / min(c, pos_len) ).
+ * These are bit-identical to the host's per-user values.  sums: [FR_TOPK_METRICS][n_cut] in the order recall, recall2,
+ * ndcg, precision, map, then sum pos_len.  per_user (or NULL): [n][FR_TOPK_METRICS][n_cut] fp64.  pos_len < 1 gives NaN.
+ *
+ * fr_by_user_metrics: user r owns scores[ptr[r] .. ptr[r+1]), its first n_pos[r] entries are the positives.  Per user:
+ *   AUC = #{(i positive, j negative) : s_j < s_i} / (n_pos * neg_num)   (neg_num as given, like the reference);
+ *   rank_i = #{j : s_j > s_i} + #{j > i : s_j == s_i}, the position of i in np.argsort(s, kind="stable")[::-1] --
+ *   the host's default (unstable) argsort agrees with it wherever a positive's score ties no other score;
+ *   Recall@c = #{i : rank_i < c} / n_pos, NDCG@c = sum_{rank_i < c} 1/log2(rank_i + 2) / sum_{t < min(c, L, n_pos)}
+ *   1/log2(t + 2) (fp64, L = segment length).  Cutoffs 1..64.  sums: [AUC, Recall@c_0.., NDCG@c_0..]; per_user (or
+ *   NULL): [n][1 + 2 n_cut] fp64.  A user with n_pos < 1 or n_pos > L gives NaN.
+ */
+#define FR_EVAL_MAX_CUTOFFS 8
+#define FR_TOPK_METRICS 5
+int64_t fr_eval_metrics_ws_bytes(void);
+int fr_topk_metrics(const void *top, int32_t idx64, int64_t n, int32_t K, const int64_t *pos_ptr, const int32_t *pos_idx,
+                    const int32_t *pos_len, const int32_t *cutoffs_host, int32_t n_cut, const float *disc,
+                    const float *ideal, double *sums, double *per_user, void *ws, void *stream);
+int fr_by_user_metrics(const float *scores, const int64_t *ptr, const int32_t *n_pos, int64_t n, int32_t neg_num,
+                       const int32_t *cutoffs_host, int32_t n_cut, double *sums, double *per_user, void *ws,
+                       void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -90,6 +90,9 @@ SIGNATURES = {
     "fr_schgn_score": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _p, _p, _i32, _i32, _p, _p]),
     "fr_schgn_score_topk_ws_bytes": (_i64, [_i32, _i32, _i32]),
     "fr_schgn_score_topk": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _p, _p, _i32, _i32, _p, _p, _p, _i32, _p, _p, _p, _p]),
+    "fr_eval_metrics_ws_bytes": (_i64, []),
+    "fr_topk_metrics": (C.c_int, [_p, _i32, _i64, _i32, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p]),
+    "fr_by_user_metrics": (C.c_int, [_p, _p, _p, _i64, _i32, _p, _i32, _p, _p, _p, _p]),
 }
 
 class SpmmTask(C.Structure):

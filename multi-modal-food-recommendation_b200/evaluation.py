@@ -260,17 +260,25 @@ def full_sort_topk(user_all: torch.Tensor, item_all: torch.Tensor, users: torch.
 
 
 def evaluate_full_sort(model, eval_users, pos_items, topk=(5, 10, 20, 50), metrics=("recall", "ndcg", "precision", "map"),
-                       hist: HistoryCSR | None = None, batch_users: int = 65536):
+                       hist: HistoryCSR | None = None, batch_users: int = 65536, device_metrics: bool = False):
     """`Trainer.evaluate` (FoodRec/common/trainer.py:476-503): rank every eval user against all items and
     score with the reference's metric definitions.  Dot-product models propagate once and rank on the
-    tensor cores; a model with its own `full_sort_topk` (SCHGN: fused pair scorer) is asked directly."""
+    tensor cores; a model with its own `full_sort_topk` (SCHGN: fused pair scorer) is asked directly.
+
+    `device_metrics=True` computes the metrics on the GPU (`metrics.topk_metrics_device`): the top-K indices stay
+    there and are returned as a device tensor; `pos_items` may then be a `metrics.ItemSets` built once per split."""
     from . import metrics as M
+    if not device_metrics and isinstance(pos_items, M.ItemSets):
+        raise ValueError("an ItemSets is the device form of pos_items: pass device_metrics=True, or the lists")
     model.eval()
     with torch.no_grad():
         if hasattr(model, "full_sort_topk"):
             dev = next(model.parameters()).device
             users = torch.as_tensor(np.asarray(eval_users), device=dev)
-            top = model.full_sort_topk(users, max(topk), hist=hist)[1].cpu().numpy()
+            top = model.full_sort_topk(users, max(topk), hist=hist)[1]
+            if device_metrics:
+                return M.topk_metrics_device(top, pos_items, metrics=metrics, topk=topk), top
+            top = top.cpu().numpy()
             return M.topk_metrics(top, pos_items, metrics=metrics, topk=topk), top
         user_all, item_all = model._tables()
         users = torch.as_tensor(np.asarray(eval_users), device=user_all.device)
@@ -280,7 +288,10 @@ def evaluate_full_sort(model, eval_users, pos_items, topk=(5, 10, 20, 50), metri
             _, idx = full_sort_topk(user_all, item_all, users[s:s + batch_users], max(topk), hist=hist,
                                     B_bf16=item_bf16, b_max_norm=bmax, index_dtype=torch.int32)
             tops.append(idx)
-        top = torch.cat(tops, 0).cpu().numpy().astype(np.int64)
+        top = torch.cat(tops, 0)
+        if device_metrics:
+            return M.topk_metrics_device(top, pos_items, metrics=metrics, topk=topk), top
+        top = top.cpu().numpy().astype(np.int64)
     return M.topk_metrics(top, pos_items, metrics=metrics, topk=topk), top
 
 
@@ -384,7 +395,7 @@ def schgn_pair_scores(*, user_final, user_key, user_comp, user_hidden, W_item, W
     return scores if topk is None else (out_v, out_i)
 
 
-def evaluate_by_user(model, users, cand_ptr, cand_items, n_pos, neg_num: int = 500):
+def evaluate_by_user(model, users, cand_ptr, cand_items, n_pos, neg_num: int = 500, device_metrics: bool = False):
     """The reference's default evaluation (`eval_by_user: True`): every user is scored against its
     positives followed by `neg_num` sampled negatives (FoodRec/common/trainer.py:231-282,
     utils/dataloader.py:228-302).  The reference propagates once and then, PER USER, calls
@@ -392,7 +403,8 @@ def evaluate_by_user(model, users, cand_ptr, cand_items, n_pos, neg_num: int = 5
     are scored by one `fr_pair_scores` launch and read back once.
 
     `users [n]`, `cand_ptr [n+1]`, `cand_items [cand_ptr[-1]]` (positives first for each user), `n_pos [n]`
-    are host arrays.  Returns the reference's metric dict."""
+    are host arrays.  Returns the reference's metric dict.  `device_metrics=True` computes it on the GPU
+    (`metrics.by_user_metrics_device`) and returns the scores as a device tensor instead of copying them back."""
     from . import metrics as M, ops
     users = np.asarray(users, dtype=np.int64)
     cand_ptr = np.asarray(cand_ptr, dtype=np.int64)
@@ -403,5 +415,7 @@ def evaluate_by_user(model, users, cand_ptr, cand_items, n_pos, neg_num: int = 5
         dev = user_all.device
         rep = np.repeat(users, np.diff(cand_ptr))
         scores = ops.pair_scores(user_all, item_all, torch.from_numpy(rep).to(dev), torch.from_numpy(cand_items).to(dev))
+        if device_metrics:
+            return M.by_user_metrics_device(scores, cand_ptr, np.asarray(n_pos), neg_num), scores
         scores = scores.cpu().numpy()
     return M.by_user_metrics(scores, cand_ptr, np.asarray(n_pos), neg_num), scores
