@@ -320,6 +320,35 @@ int fr_schgn_score_topk(const float *user_final, const float *user_hidden, int32
                         const float *W_prod, const float *w_out, const float *comps, const float *att, const float *logits,
                         int32_t n_items, int32_t d, const int64_t *user_ids, const int64_t *hist_ptr,
                         const int32_t *hist_idx, int32_t k, void *ws, float *out_val, int64_t *out_idx, void *stream);
+/* The same scorer over per-user candidate lists (by-user evaluation, FoodRec/common/trainer.py:231-282: each user's
+ * held-out positives, then sampled negatives, scored as ONE `inference_by_user` batch).  User u of the call owns pairs
+ * q = ptr[u] - ptr[0] .. ptr[u+1] - ptr[0] - 1 (ptr int64 [nu + 1], strictly increasing: no empty list; n_pairs =
+ * ptr[nu] - ptr[0]); pair q is candidate items[q] (int32).  The component softmax groups each list's own logits as the
+ * reference does with b = L, the list length: row r takes flat entries 4r .. 4r+3 of the list's component-major [4, L]
+ * block, so it depends on the list's order and length.  Item-side tables as above, user rows [nu, 64].
+ *   fr_schgn_attend_pairs: att [n_pairs, 64] and logits [4 n_pairs] (list of user u at 4 (ptr[u] - ptr[0]), [4, L]).
+ *     Groups the pairs by item on the device (ws: fr_schgn_attend_pairs_ws_bytes(nu, n_pairs, n_items) bytes,
+ *     16-byte aligned).  The lists are checked on the device: *status (device int32, zeroed by the caller) gets
+ *     FR_PAIRS_BAD_PTR when a list is empty, ptr does not increase or ptr[nu] - ptr[0] != n_pairs, and
+ *     FR_PAIRS_BAD_ITEM for an item outside [0, n_items).  Bad lists / pairs are skipped, never dereferenced; their
+ *     outputs are undefined, so the caller reads *status before it uses any score.  A bad ptr can make the lists that
+ *     pass their own check overlap, so once FR_PAIRS_BAD_PTR is set nothing after the check is computed: att and
+ *     logits are left as they were and no byte past the workspace's grp array is written.
+ *   fr_schgn_score_pairs: scores [n_pairs] from the att / logits of fr_schgn_attend_pairs on the same ptr / items.
+ * Float tables 16-byte aligned; at most 2^31 - 1 pairs per call. */
+#define FR_PAIRS_BAD_PTR 1
+#define FR_PAIRS_BAD_ITEM 2
+int64_t fr_schgn_attend_pairs_ws_bytes(int32_t nu, int64_t n_pairs, int32_t n_items);
+int fr_schgn_attend_pairs(const float *user_key, const float *user_comp, int32_t nu, const int64_t *ptr,
+                          const int32_t *items, int64_t n_pairs, const int32_t *codes, int32_t slots, const int32_t *nums,
+                          int32_t n_items, const float *ingre_key, const float *ingre_final, const float *ingre_comp,
+                          const float *img_key, const float *comp_keys, const float *h_ingre, const float *h_comp,
+                          int32_t d, void *ws, int64_t ws_bytes, float *att, float *logits, int32_t *status,
+                          void *stream);
+int fr_schgn_score_pairs(const float *user_final, const float *user_hidden, int32_t nu, const int64_t *ptr,
+                         const int32_t *items, int64_t n_pairs, const float *W_item, const float *W_prod,
+                         const float *w_out, const float *comps, const float *att, const float *logits, int32_t n_items,
+                         int32_t d, float *scores, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Row-partitioned multi-GPU propagation over peer memory (one process per GPU, one NVLink/NVSwitch node).

@@ -357,6 +357,356 @@ schgn_merge_topk_kernel(const unsigned long long *__restrict__ cand, int n_cand,
     }
 }
 
+// ------------------------------------------------------------------------------------------------ candidate lists
+// By-user evaluation: user u of a block has its own candidate list; pair q = ptr[u] - ptr[0] + k is its k-th candidate
+// items[q].  The same per-pair arithmetic as above, with two changes:
+//   * attend runs item-major over the block's pairs grouped by candidate item (a counting sort: count, scan, scatter),
+//     one warp per item and 16 of its pairs per pass, so the gathered ingredient rows and their e^{2a} factors are
+//     reused across the users that hold the item, as schgn_attend_kernel reuses them across a fixed 16-user block;
+//   * the component softmax groups the logits of each user's OWN list: with L = the list's length, row r reads flat
+//     entries 4r .. 4r+3 of the list's component-major [4, L] logit block, which is what the reference computes when
+//     the list is scored as one batch (`.view(b, -1)` with b = L, schgn.py:198).
+// A pair's result does not depend on which pass or slot it lands in (the reduce16 tree is the same for every slot), so
+// the atomics' ordering of the scatter leaves every score bit-reproducible.
+constexpr int PL_WARPS = 8;   // users per CTA of the count / scatter passes (one warp each)
+
+// User u's pair range [b, e), or false when it is empty or leaves [0, n_pairs) (ptr not increasing), or the last list
+// does not end at n_pairs.  This check is per list: with a decreasing ptr the lists that pass it can overlap (ptr =
+// [0, 4, 2, 6] passes [0, 4) and [2, 6)), and the per-item counts then exceed n_pairs.  So once the count kernel has
+// set FR_PAIRS_BAD_PTR for any list, the scatter and attend launches that follow it on the stream do nothing.
+__device__ __forceinline__ bool list_range(const int64_t *ptr, int u, int32_t nu, int64_t n_pairs, int64_t &b, int64_t &e) {
+    b = ptr[u] - ptr[0];
+    e = ptr[u + 1] - ptr[0];
+    return b >= 0 && e > b && e <= n_pairs && (u < nu - 1 || e == n_pairs);
+}
+__device__ __forceinline__ bool item_ok(int it, int32_t n_items) { return it >= 0 && it < n_items; }
+
+// Validation + per-item pair counts.  status |= FR_PAIRS_BAD_PTR / FR_PAIRS_BAD_ITEM.
+__global__ void __launch_bounds__(PL_WARPS * 32)
+pairs_count_kernel(const int64_t *__restrict__ ptr, int32_t nu, int64_t n_pairs, const int32_t *__restrict__ items,
+                   int32_t n_items, int32_t *__restrict__ cnt, int32_t *__restrict__ status) {
+    const int u = blockIdx.x * PL_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (u >= nu) return;
+    int64_t b, e;
+    if (!list_range(ptr, u, nu, n_pairs, b, e)) {
+        if (lane == 0) atomicOr(status, FR_PAIRS_BAD_PTR);
+        return;
+    }
+    for (int64_t q = b + lane; q < e; q += 32) {
+        const int it = items[q];
+        if (item_ok(it, n_items)) atomicAdd(cnt + it, 1);
+        else atomicOr(status, FR_PAIRS_BAD_ITEM);
+    }
+}
+
+// Exclusive scan of cnt[0, n) in one CTA -> cnt (item_ptr, with cnt[n] = total) and cursor (a copy for the scatter).
+__global__ void __launch_bounds__(1024) pairs_scan_kernel(int32_t *__restrict__ cnt, int32_t *__restrict__ cursor, int32_t n) {
+    __shared__ int32_t s_warp[32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int per = (n + 1023) / 1024, lo = min(n, tid * per), hi = min(n, lo + per);
+    int sum = 0;
+    for (int i = lo; i < hi; ++i) sum += cnt[i];
+    int x = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= o) x += y;
+    }
+    if (lane == 31) s_warp[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+        int w = s_warp[lane];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, w, o);
+            if (lane >= o) w += y;
+        }
+        s_warp[lane] = w;
+    }
+    __syncthreads();
+    int run = x - sum + (warp ? s_warp[warp - 1] : 0);
+    for (int i = lo; i < hi; ++i) {
+        const int c = cnt[i];
+        cnt[i] = cursor[i] = run;
+        run += c;
+    }
+    if (tid == 1023) cnt[n] = run;
+}
+
+// Pairs into their item's group as (pair, user); and the user factors e^{2 user_key}, e^{2 user_comp} -> uexp [nu][2][64].
+__global__ void __launch_bounds__(PL_WARPS * 32)
+pairs_scatter_kernel(const int64_t *__restrict__ ptr, int32_t nu, int64_t n_pairs, const int32_t *__restrict__ items,
+                     int32_t n_items, const float *__restrict__ user_key, const float *__restrict__ user_comp,
+                     const int32_t *__restrict__ status, int32_t *__restrict__ cursor, int2 *__restrict__ grp,
+                     float *__restrict__ uexp) {
+    const int u = blockIdx.x * PL_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (u >= nu || (*status & FR_PAIRS_BAD_PTR)) return;     // lists may overlap: the group offsets are not valid
+    const int c2 = 2 * lane;
+    const float2 k = *reinterpret_cast<const float2 *>(user_key + (size_t)u * D + c2);
+    const float2 c = *reinterpret_cast<const float2 *>(user_comp + (size_t)u * D + c2);
+    *reinterpret_cast<float2 *>(uexp + (size_t)u * 2 * D + c2) = make_float2(exp2x(k.x), exp2x(k.y));
+    *reinterpret_cast<float2 *>(uexp + (size_t)u * 2 * D + D + c2) = make_float2(exp2x(c.x), exp2x(c.y));
+    int64_t b, e;
+    if (!list_range(ptr, u, nu, n_pairs, b, e)) return;
+    for (int64_t q = b + lane; q < e; q += 32)
+        if (item_ok(items[q], n_items)) grp[atomicAdd(cursor + items[q], 1)] = make_int2((int)q, u);
+}
+
+struct AttendPairsParams {
+    const int64_t *ptr;
+    const int32_t *item_ptr;
+    const int2 *grp;
+    const float *uexp;
+    const int32_t *codes, *nums;
+    const float *ingre_key, *ingre_final, *ingre_comp, *img_key, *comp_keys, *h_ingre, *h_comp;
+    float *att, *logits;
+    const int32_t *status;
+    int32_t n_items, slots;
+};
+
+// schgn_attend_kernel's two passes and component logits for the pairs of one item, 16 per pass; writes att [q] and
+// the logits into each pair's list block: logits[4 (ptr[u] - ptr[0]) + comp L + k].
+__global__ void __launch_bounds__(ATT_WARPS * 32, 2) schgn_attend_pairs_kernel(const AttendPairsParams p) {
+    __shared__ float s_u[ATT_WARPS][UB][D];   // per warp: e^{2 user_key} of the pass's users, then their e^{2 user_comp}
+    __shared__ float s_logit[ATT_WARPS][UB][MAX_SLOTS];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int item = blockIdx.x * ATT_WARPS + warp;
+    if (item >= p.n_items || (*p.status & FR_PAIRS_BAD_PTR)) return;   // grp was not filled
+    const int g0 = p.item_ptr[item], g1 = p.item_ptr[item + 1];
+    if (g0 == g1) return;
+    const int n = max(0, min(p.nums[item], p.slots));
+    const int code = lane < p.slots ? p.codes[(size_t)item * p.slots + lane] : 0;
+    const int c2 = 2 * lane;
+    const float2 pi = *reinterpret_cast<const float2 *>(p.img_key + (size_t)item * D + c2);
+    const float2 hi = *reinterpret_cast<const float2 *>(p.h_ingre + c2);
+    const float2 hc = *reinterpret_cast<const float2 *>(p.h_comp + c2);
+    const float hi_sum = hi.x + hi.y, hc_sum = hc.x + hc.y;
+    float(&su)[UB][D] = s_u[warp];
+
+    for (int g = g0; g < g1; g += UB) {
+        // lanes 2s and 2s+1 own slot s of the pass; slots past the group's end repeat slot 0 and write nothing
+        const bool valid = g + (lane >> 1) < g1;
+        const int2 pr = p.grp[valid ? g + (lane >> 1) : g];
+        __syncwarp();                                  // the previous pass has finished reading su
+#pragma unroll
+        for (int s = 0; s < UB; ++s) {
+            const int us = __shfl_sync(0xffffffffu, pr.y, 2 * s);
+            *reinterpret_cast<float2 *>(&su[s][c2]) = __ldg(reinterpret_cast<const float2 *>(p.uexp + (size_t)us * 2 * D + c2));
+        }
+        __syncwarp();
+
+        // pass 1: attention logits a[s][j]
+        for (int j = 0; j < n; ++j) {
+            const int c = __shfl_sync(0xffffffffu, code, j);
+            const float2 pe = __ldg(reinterpret_cast<const float2 *>(p.ingre_key + (size_t)c * D + c2));
+            const float ex = exp2x(pe.x + pi.x), ey = exp2x(pe.y + pi.y);
+            float v[UB];
+#pragma unroll
+            for (int s = 0; s < UB; ++s) {
+                const float2 uk = *reinterpret_cast<const float2 *>(&su[s][c2]);
+                v[s] = fmaf(-2.0f, fmaf(hi.x, inv1p(ex, uk.x), hi.y * inv1p(ey, uk.y)), hi_sum);
+            }
+            const float tot = reduce16(v, lane);
+            if (!(lane & 1)) s_logit[warp][lane >> 1][j] = tot;
+        }
+        __syncwarp();
+#pragma unroll
+        for (int s = 0; s < UB; ++s) {
+            const int us = __shfl_sync(0xffffffffu, pr.y, 2 * s);
+            *reinterpret_cast<float2 *>(&su[s][c2]) =
+                __ldg(reinterpret_cast<const float2 *>(p.uexp + (size_t)us * 2 * D + D + c2));
+        }
+
+        // softmax over the recipe's real ingredients; lane j keeps A[s][j]
+        float A[UB];
+#pragma unroll
+        for (int s = 0; s < UB; ++s) {
+            const float x = lane < n ? s_logit[warp][s][lane] : -INFINITY;
+            float m = x;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+            const float e = lane < n ? expf(x - m) : 0.0f;
+            const float sum = fr::warp_sum(e);
+            A[s] = n > 0 ? e / sum : 0.0f;
+        }
+
+        // pass 2: attended ingredient row and its image under W_att_comp's component half
+        float2 att[UB], q[UB];
+#pragma unroll
+        for (int s = 0; s < UB; ++s) att[s] = q[s] = make_float2(0.0f, 0.0f);
+        for (int j = 0; j < n; ++j) {
+            const int c = __shfl_sync(0xffffffffu, code, j);
+            const float2 ef = __ldg(reinterpret_cast<const float2 *>(p.ingre_final + (size_t)c * D + c2));
+            const float2 qe = __ldg(reinterpret_cast<const float2 *>(p.ingre_comp + (size_t)c * D + c2));
+#pragma unroll
+            for (int s = 0; s < UB; ++s) {
+                const float w = __shfl_sync(0xffffffffu, A[s], j);
+                att[s].x = fmaf(w, ef.x, att[s].x);
+                att[s].y = fmaf(w, ef.y, att[s].y);
+                q[s].x = fmaf(w, qe.x, q[s].x);
+                q[s].y = fmaf(w, qe.y, q[s].y);
+            }
+        }
+#pragma unroll
+        for (int s = 0; s < UB; ++s) {
+            const int qs = __shfl_sync(0xffffffffu, pr.x, 2 * s);
+            if (g + s < g1) *reinterpret_cast<float2 *>(p.att + (size_t)qs * D + c2) = att[s];
+        }
+        __syncwarp();                                  // su holds e^{2 user_comp} for every lane
+
+        // component logits, reference order: item id, attended ingredients, image, health (the item's factors are
+        // recomputed per pass: keeping them live across passes costs spills at two CTAs per SM)
+        const float *ck = p.comp_keys + (size_t)item * 3 * D + c2;
+        float2 k_item = *reinterpret_cast<const float2 *>(ck);
+        float2 k_img = *reinterpret_cast<const float2 *>(ck + D);
+        float2 k_hl = *reinterpret_cast<const float2 *>(ck + 2 * D);
+        k_item = make_float2(exp2x(k_item.x), exp2x(k_item.y));
+        k_img = make_float2(exp2x(k_img.x), exp2x(k_img.y));
+        k_hl = make_float2(exp2x(k_hl.x), exp2x(k_hl.y));
+        const int64_t ub = p.ptr[pr.y] - p.ptr[0], L = p.ptr[pr.y + 1] - p.ptr[pr.y];
+        float *lg = p.logits + 4 * ub + (pr.x - ub);
+#pragma unroll
+        for (int comp = 0; comp < 4; ++comp) {
+            float v[UB];
+#pragma unroll
+            for (int s = 0; s < UB; ++s) {
+                const float2 uc = *reinterpret_cast<const float2 *>(&su[s][c2]);
+                const float2 k = comp == 0   ? k_item
+                                 : comp == 1 ? make_float2(exp2x(q[s].x), exp2x(q[s].y))
+                                 : comp == 2 ? k_img
+                                             : k_hl;
+                v[s] = fmaf(-2.0f, fmaf(hc.x, inv1p(k.x, uc.x), hc.y * inv1p(k.y, uc.y)), hc_sum);
+            }
+            const float tot = reduce16(v, lane);
+            if (!(lane & 1) && valid) lg[comp * L] = tot;
+        }
+    }
+}
+
+struct ScorePairsParams {
+    const int64_t *ptr;
+    const int32_t *items;
+    const float *user_final, *user_hidden, *W_item, *W_prod, *w_out, *comps, *att, *logits;
+    float *scores;
+    int64_t n_pairs;
+    int32_t nu, n_items;
+};
+
+// One CTA per user: M_u built once in shared memory, then the user's list in tiles of SC_ITEMS candidates with the
+// tile body of schgn_score_kernel.  Candidate r's component weights: softmax of logits[4 (ptr[u] - ptr[0]) + 4r ..+3].
+__global__ void __launch_bounds__(SC_THREADS) schgn_score_pairs_kernel(const ScorePairsParams p) {
+    extern __shared__ __align__(16) float smem[];
+    float *sX = smem;                    // [SC_ITEMS][XS]   x rows of the tile
+    float *sM = sX + SC_ITEMS * XS;      // [D][D]           M_u = W_item + W_prod diag(u_final)
+    float *sH = sM + D * D;              // [D]              user_hidden[u]
+    float *sW = sH + D;                  // [D]              w_out
+    float *sB = sW + D;                  // [SC_ITEMS][4]    component softmax weights
+    const int u = blockIdx.x, tid = threadIdx.x;
+    int64_t ub, ue;
+    if (!list_range(p.ptr, u, p.nu, p.n_pairs, ub, ue)) return;      // reported by fr_schgn_attend_pairs
+    const int L = (int)(ue - ub);
+    for (int t = tid; t < D * D; t += SC_THREADS)
+        sM[t] = fmaf(p.W_prod[t], p.user_final[(size_t)u * D + t % D], p.W_item[t]);
+    if (tid < D) {
+        sH[tid] = p.user_hidden[(size_t)u * D + tid];
+        sW[tid] = p.w_out[tid];
+    }
+    const float *lg = p.logits + 4 * ub;
+    const int32_t *it = p.items + ub;
+    const float *att = p.att + ub * D;
+    for (int base = 0; base < L; base += SC_ITEMS) {
+        if (base) __syncthreads();       // every thread holds its previous x rows in registers: the tile is free
+#pragma unroll
+        for (int t = 0; t < IPT; ++t) {
+            const int r = min(base + tid + t * SC_THREADS, L - 1);
+            const float4 l = *reinterpret_cast<const float4 *>(lg + (size_t)4 * r);
+            const float m = fmaxf(fmaxf(l.x, l.y), fmaxf(l.z, l.w));
+            const float e0 = expf(l.x - m), e1 = expf(l.y - m), e2 = expf(l.z - m), e3 = expf(l.w - m);
+            const float inv = 1.0f / (e0 + e1 + e2 + e3);
+            *reinterpret_cast<float4 *>(sB + 4 * (tid + t * SC_THREADS)) = make_float4(e0 * inv, e1 * inv, e2 * inv, e3 * inv);
+        }
+        __syncthreads();
+        {
+            const int sub = (tid & 15) * 4, rr = tid >> 4;
+#pragma unroll 4
+            for (int row = rr; row < SC_ITEMS; row += SC_THREADS / 16) {
+                const int r = min(base + row, L - 1);
+                const int item = min(max(it[r], 0), p.n_items - 1);   // a bad id is reported by fr_schgn_attend_pairs
+                const float4 b = *reinterpret_cast<const float4 *>(sB + 4 * row);
+                const float *cr = p.comps + (size_t)item * 3 * D + sub;
+                const float4 ci = fr::ldg_f4(cr), cm = fr::ldg_f4(cr + D), ch = fr::ldg_f4(cr + 2 * D);
+                const float4 ca = fr::ldg_f4(att + (size_t)r * D + sub);
+                float4 x;
+                x.x = b.x * ci.x + b.y * ca.x + b.z * cm.x + b.w * ch.x;
+                x.y = b.x * ci.y + b.y * ca.y + b.z * cm.y + b.w * ch.y;
+                x.z = b.x * ci.z + b.y * ca.z + b.z * cm.z + b.w * ch.z;
+                x.w = b.x * ci.w + b.y * ca.w + b.z * cm.w + b.w * ch.w;
+                *reinterpret_cast<float4 *>(sX + row * XS + sub) = x;
+            }
+        }
+        __syncthreads();
+        float x[IPT][D];
+#pragma unroll
+        for (int t = 0; t < IPT; ++t)
+#pragma unroll
+            for (int d = 0; d < D; d += 4) {
+                const float4 v = *reinterpret_cast<const float4 *>(sX + (tid + t * SC_THREADS) * XS + d);
+                x[t][d] = v.x, x[t][d + 1] = v.y, x[t][d + 2] = v.z, x[t][d + 3] = v.w;
+            }
+        float score[IPT];
+#pragma unroll
+        for (int t = 0; t < IPT; ++t) score[t] = 0.0f;
+#pragma unroll 2
+        for (int e = 0; e < D; ++e) {
+            float h[IPT][4];
+#pragma unroll
+            for (int t = 0; t < IPT; ++t) h[t][0] = sH[e], h[t][1] = h[t][2] = h[t][3] = 0.0f;
+#pragma unroll
+            for (int d = 0; d < D; d += 4) {
+                const float4 m = *reinterpret_cast<const float4 *>(sM + e * D + d);
+#pragma unroll
+                for (int t = 0; t < IPT; ++t) {
+                    h[t][0] = fmaf(m.x, x[t][d + 0], h[t][0]);
+                    h[t][1] = fmaf(m.y, x[t][d + 1], h[t][1]);
+                    h[t][2] = fmaf(m.z, x[t][d + 2], h[t][2]);
+                    h[t][3] = fmaf(m.w, x[t][d + 3], h[t][3]);
+                }
+            }
+            const float w = sW[e];
+#pragma unroll
+            for (int t = 0; t < IPT; ++t)
+                score[t] = fmaf(w, fmaxf((h[t][0] + h[t][1]) + (h[t][2] + h[t][3]), 0.0f), score[t]);
+        }
+#pragma unroll
+        for (int t = 0; t < IPT; ++t) {
+            const int r = base + tid + t * SC_THREADS;
+            if (r < L) p.scores[ub + r] = score[t];
+        }
+    }
+}
+
+// workspace of fr_schgn_attend_pairs: cnt [n_items + 1] | cursor [n_items] | grp [n_pairs] | uexp [nu][2][64]
+struct PairsWs {
+    int32_t *cnt, *cursor;
+    int2 *grp;
+    float *uexp;
+    int64_t bytes;
+};
+inline int64_t align16(int64_t b) { return (b + 15) & ~int64_t(15); }
+inline PairsWs pairs_ws(void *base, int32_t nu, int64_t n_pairs, int32_t n_items) {
+    char *b = static_cast<char *>(base);
+    PairsWs w;
+    int64_t off = 0;
+    w.cnt = reinterpret_cast<int32_t *>(b + off), off += align16(4 * ((int64_t)n_items + 1));
+    w.cursor = reinterpret_cast<int32_t *>(b + off), off += align16(4 * (int64_t)n_items);
+    w.grp = reinterpret_cast<int2 *>(b + off), off += align16(8 * n_pairs);
+    w.uexp = reinterpret_cast<float *>(b + off), off += (int64_t)nu * 2 * D * 4;
+    w.bytes = off;
+    return w;
+}
+
+inline bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
+
 }  // namespace
 
 extern "C" int fr_schgn_attend(const float *user_key, const float *user_comp, int32_t nu, const int32_t *codes,
@@ -443,4 +793,84 @@ extern "C" int fr_schgn_score_topk(const float *user_final, const float *user_hi
     fr::LaunchTimer timer("schgn_merge_topk", st);
     schgn_merge_topk_kernel<<<nu, 256, 0, st>>>(p.cand, n_blk * k, k, out_val, out_idx);
     return fr::check_launch("fr_schgn_score_topk(merge)");
+}
+
+extern "C" int64_t fr_schgn_attend_pairs_ws_bytes(int32_t nu, int64_t n_pairs, int32_t n_items) {
+    if (nu < 0 || n_pairs < 0 || n_items < 0) return -1;
+    return pairs_ws(nullptr, nu, n_pairs, n_items).bytes;
+}
+
+extern "C" int fr_schgn_attend_pairs(const float *user_key, const float *user_comp, int32_t nu, const int64_t *ptr,
+                                     const int32_t *items, int64_t n_pairs, const int32_t *codes, int32_t slots,
+                                     const int32_t *nums, int32_t n_items, const float *ingre_key,
+                                     const float *ingre_final, const float *ingre_comp, const float *img_key,
+                                     const float *comp_keys, const float *h_ingre, const float *h_comp, int32_t d,
+                                     void *ws, int64_t ws_bytes, float *att, float *logits, int32_t *status,
+                                     void *stream) {
+    FR_REQUIRE(d == D, "fr_schgn_attend_pairs: embedding width %d unsupported (the model fixes 64)", d);
+    FR_REQUIRE(nu >= 0 && n_items >= 1 && slots >= 1 && slots <= MAX_SLOTS,
+               "fr_schgn_attend_pairs: bad extents (nu=%d, n_items=%d, slots=%d; at most %d slots)", nu, n_items, slots,
+               MAX_SLOTS);
+    if (nu == 0) return FR_OK;
+    FR_REQUIRE(n_pairs >= nu && n_pairs <= INT32_MAX,
+               "fr_schgn_attend_pairs: %lld pairs for %d users (every list non-empty, at most 2^31 - 1 pairs per call)",
+               (long long)n_pairs, nu);
+    FR_REQUIRE(user_key && user_comp && ptr && items && codes && nums && ingre_key && ingre_final && ingre_comp &&
+                   img_key && comp_keys && h_ingre && h_comp && ws && att && logits && status,
+               "fr_schgn_attend_pairs: null pointer");
+    FR_REQUIRE(aligned16(user_key) && aligned16(user_comp) && aligned16(ingre_key) && aligned16(ingre_final) &&
+                   aligned16(ingre_comp) && aligned16(img_key) && aligned16(comp_keys) && aligned16(h_ingre) &&
+                   aligned16(h_comp) && aligned16(ws) && aligned16(att) && aligned16(logits) && ((uintptr_t)ptr & 7) == 0 &&
+                   ((uintptr_t)items & 3) == 0 && ((uintptr_t)status & 3) == 0,
+               "fr_schgn_attend_pairs: tables must be 16-byte aligned (ptr 8-byte, items / status 4-byte)");
+    const PairsWs w = pairs_ws(ws, nu, n_pairs, n_items);
+    FR_REQUIRE(ws_bytes >= w.bytes, "fr_schgn_attend_pairs: workspace of %lld bytes, %lld needed", (long long)ws_bytes,
+               (long long)w.bytes);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int ublocks = (nu + PL_WARPS - 1) / PL_WARPS;
+    {
+        fr::LaunchTimer timer("schgn_pairs_group", st);
+        if (cudaMemsetAsync(w.cnt, 0, 4 * ((int64_t)n_items + 1), st) != cudaSuccess)
+            return fr::check_launch("fr_schgn_attend_pairs (memset)");
+        pairs_count_kernel<<<ublocks, PL_WARPS * 32, 0, st>>>(ptr, nu, n_pairs, items, n_items, w.cnt, status);
+        if (int rc = fr::check_launch("fr_schgn_attend_pairs(count)")) return rc;
+        pairs_scan_kernel<<<1, 1024, 0, st>>>(w.cnt, w.cursor, n_items);
+        if (int rc = fr::check_launch("fr_schgn_attend_pairs(scan)")) return rc;
+        pairs_scatter_kernel<<<ublocks, PL_WARPS * 32, 0, st>>>(ptr, nu, n_pairs, items, n_items, user_key, user_comp,
+                                                                 status, w.cursor, w.grp, w.uexp);
+        if (int rc = fr::check_launch("fr_schgn_attend_pairs(scatter)")) return rc;
+    }
+    AttendPairsParams p{ptr,     w.cnt,       w.grp,      w.uexp,  codes,     nums,   ingre_key, ingre_final,
+                        ingre_comp, img_key, comp_keys, h_ingre, h_comp, att, logits, status, n_items, slots};
+    fr::LaunchTimer timer("schgn_attend_pairs", st);
+    schgn_attend_pairs_kernel<<<(n_items + ATT_WARPS - 1) / ATT_WARPS, ATT_WARPS * 32, 0, st>>>(p);
+    return fr::check_launch("fr_schgn_attend_pairs");
+}
+
+extern "C" int fr_schgn_score_pairs(const float *user_final, const float *user_hidden, int32_t nu, const int64_t *ptr,
+                                    const int32_t *items, int64_t n_pairs, const float *W_item, const float *W_prod,
+                                    const float *w_out, const float *comps, const float *att, const float *logits,
+                                    int32_t n_items, int32_t d, float *scores, void *stream) {
+    FR_REQUIRE(d == D, "fr_schgn_score_pairs: embedding width %d unsupported (the model fixes 64)", d);
+    FR_REQUIRE(nu >= 0 && n_items >= 1, "fr_schgn_score_pairs: bad extents (nu=%d, n_items=%d)", nu, n_items);
+    if (nu == 0) return FR_OK;
+    FR_REQUIRE(n_pairs >= nu && n_pairs <= INT32_MAX, "fr_schgn_score_pairs: %lld pairs for %d users", (long long)n_pairs, nu);
+    FR_REQUIRE(user_final && user_hidden && ptr && items && W_item && W_prod && w_out && comps && att && logits && scores,
+               "fr_schgn_score_pairs: null pointer");
+    FR_REQUIRE(aligned16(user_final) && aligned16(user_hidden) && aligned16(W_item) && aligned16(W_prod) &&
+                   aligned16(w_out) && aligned16(comps) && aligned16(att) && aligned16(logits) &&
+                   ((uintptr_t)ptr & 7) == 0 && ((uintptr_t)items & 3) == 0 && ((uintptr_t)scores & 3) == 0,
+               "fr_schgn_score_pairs: tables must be 16-byte aligned (ptr 8-byte, items / scores 4-byte)");
+    ScorePairsParams p{ptr, items, user_final, user_hidden, W_item, W_prod, w_out, comps, att, logits, scores, n_pairs,
+                       nu, n_items};
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    fr::LaunchTimer timer("schgn_score_pairs", st);
+    static bool configured = false;
+    if (!configured) {
+        if (cudaFuncSetAttribute(schgn_score_pairs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SC_SMEM) != cudaSuccess)
+            return fr::check_launch("fr_schgn_score_pairs (shared-memory opt-in)");
+        configured = true;
+    }
+    schgn_score_pairs_kernel<<<nu, SC_THREADS, SC_SMEM, st>>>(p);
+    return fr::check_launch("fr_schgn_score_pairs");
 }

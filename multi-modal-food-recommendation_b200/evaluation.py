@@ -395,12 +395,77 @@ def schgn_pair_scores(*, user_final, user_key, user_comp, user_hidden, W_item, W
     return scores if topk is None else (out_v, out_i)
 
 
+def schgn_by_user_scores(cand_ptr, cand_items, *, user_final, user_key, user_comp, user_hidden, W_item, W_prod, w_out,
+                         h_ingre, h_comp, codes, nums, ingre_key, ingre_final, ingre_comp, img_key, comps, comp_keys,
+                         block_pairs: int = 1 << 22):
+    """SCHGN scores of per-user candidate lists: user r (row r of the user tables) against `cand_items[cand_ptr[r]:
+    cand_ptr[r+1]]`, each list scored as the reference scores it in one `inference_by_user` batch -- the component
+    softmax groups the list's own logits (`.view(b, -1)` with b = the list length, FoodRec/models/schgn.py:198).
+    `fr_schgn_attend_pairs` + `fr_schgn_score_pairs` over the tables of `models.schgn.SCHGN._item_side`, users in blocks
+    of at most `block_pairs` pairs (one longer list forms a block alone) so the `[pairs, 64]` attended-row scratch stays
+    under ~1 GB.  `cand_ptr` [n+1] is a host array from 0 to len(cand_items); returns the flat fp32 scores [len(cand_items)]
+    in list order.  An item outside [0, n_items) raises `FoodRecError` (checked on the device: one 4-byte read-back)."""
+    dev = user_final.device
+    if dev.type != "cuda":
+        raise _lib.FoodRecError("schgn_by_user_scores needs CUDA tensors (no CPU path)")
+    f32 = [user_final, user_key, user_comp, user_hidden, W_item, W_prod, w_out, h_ingre, h_comp, ingre_key,
+           ingre_final, ingre_comp, img_key, comps, comp_keys]
+    user_final, user_key, user_comp, user_hidden, W_item, W_prod, w_out, h_ingre, h_comp, ingre_key, ingre_final, \
+        ingre_comp, img_key, comps, comp_keys = [t.detach().float().contiguous() for t in f32]
+    nu, d = user_final.shape
+    n_items, slots = codes.shape
+    if codes.dtype != torch.int32 or nums.dtype != torch.int32:
+        raise _lib.FoodRecError("ingredient codes / counts must be int32")
+    ptr = np.asarray(cand_ptr, dtype=np.int64).reshape(-1)
+    items = torch.as_tensor(cand_items).reshape(-1).to(dev)
+    if ptr.shape[0] != nu + 1:
+        raise _lib.FoodRecError(f"cand_ptr has {ptr.shape[0]} entries for {nu} users")
+    if nu == 0:
+        return torch.empty(0, dtype=torch.float32, device=dev)
+    if ptr[0] != 0 or ptr[-1] != items.numel():
+        raise _lib.FoodRecError(f"cand_ptr runs from {ptr[0]} to {ptr[-1]}, cand_items holds {items.numel()} items")
+    if (np.diff(ptr) < 1).any():
+        raise _lib.FoodRecError("every candidate list must be non-empty (cand_ptr strictly increasing)")
+    if items.dtype != torch.int32:       # an id beyond int32 must not wrap into range: map it to -1, which the kernel rejects
+        items = torch.where((items >= 0) & (items < n_items), items, -1)
+    items = items.to(torch.int32).contiguous()
+    blocks, s = [], 0
+    while s < nu:
+        e = max(s + 1, int(np.searchsorted(ptr, ptr[s] + block_pairs, side="right")) - 1)
+        blocks.append((s, min(e, nu)))
+        s = min(e, nu)
+    most = max(int(ptr[e] - ptr[s]) for s, e in blocks)
+    most_users = max(e - s for s, e in blocks)
+    ws = torch.empty(int(_L.fr_schgn_attend_pairs_ws_bytes(most_users, most, n_items)), dtype=torch.uint8, device=dev)
+    att = torch.empty(most, d, dtype=torch.float32, device=dev)
+    logits = torch.empty(4 * most, dtype=torch.float32, device=dev)
+    scores = torch.empty(items.numel(), dtype=torch.float32, device=dev)
+    ptr_d = torch.from_numpy(ptr).to(dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    st = _lib.stream_ptr()
+    for s, e in blocks:
+        n, q0, npairs = e - s, int(ptr[s]), int(ptr[e] - ptr[s])
+        _lib.check(_L.fr_schgn_attend_pairs(
+            user_key[s:].data_ptr(), user_comp[s:].data_ptr(), n, ptr_d[s:].data_ptr(), items[q0:].data_ptr(), npairs,
+            codes.data_ptr(), slots, nums.data_ptr(), n_items, ingre_key.data_ptr(), ingre_final.data_ptr(),
+            ingre_comp.data_ptr(), img_key.data_ptr(), comp_keys.data_ptr(), h_ingre.data_ptr(), h_comp.data_ptr(), d,
+            ws.data_ptr(), ws.numel(), att.data_ptr(), logits.data_ptr(), status.data_ptr(), st), "fr_schgn_attend_pairs")
+        _lib.check(_L.fr_schgn_score_pairs(
+            user_final[s:].data_ptr(), user_hidden[s:].data_ptr(), n, ptr_d[s:].data_ptr(), items[q0:].data_ptr(), npairs,
+            W_item.data_ptr(), W_prod.data_ptr(), w_out.data_ptr(), comps.data_ptr(), att.data_ptr(), logits.data_ptr(),
+            n_items, d, scores[q0:].data_ptr(), st), "fr_schgn_score_pairs")
+    if int(status.item()) != 0:          # cand_ptr was checked on the host: only an item can be out of range here
+        raise _lib.FoodRecError(f"a candidate item is outside [0, {n_items})")
+    return scores
+
+
 def evaluate_by_user(model, users, cand_ptr, cand_items, n_pos, neg_num: int = 500, device_metrics: bool = False):
     """The reference's default evaluation (`eval_by_user: True`): every user is scored against its
     positives followed by `neg_num` sampled negatives (FoodRec/common/trainer.py:231-282,
     utils/dataloader.py:228-302).  The reference propagates once and then, PER USER, calls
     `inference_fast`, copies the scores to the host and argsorts them there; here all users' candidates
-    are scored by one `fr_pair_scores` launch and read back once.
+    are scored by one `fr_pair_scores` launch and read back once.  A model with its own `by_user_scores`
+    (SCHGN: the fused pair scorer over candidate lists) is asked directly.
 
     `users [n]`, `cand_ptr [n+1]`, `cand_items [cand_ptr[-1]]` (positives first for each user), `n_pos [n]`
     are host arrays.  Returns the reference's metric dict.  `device_metrics=True` computes it on the GPU
@@ -411,10 +476,14 @@ def evaluate_by_user(model, users, cand_ptr, cand_items, n_pos, neg_num: int = 5
     cand_items = np.asarray(cand_items, dtype=np.int64)
     model.eval()
     with torch.no_grad():
-        user_all, item_all = model._tables()
-        dev = user_all.device
-        rep = np.repeat(users, np.diff(cand_ptr))
-        scores = ops.pair_scores(user_all, item_all, torch.from_numpy(rep).to(dev), torch.from_numpy(cand_items).to(dev))
+        if hasattr(model, "by_user_scores"):
+            dev = next(model.parameters()).device
+            scores = model.by_user_scores(torch.from_numpy(users).to(dev), cand_ptr, torch.from_numpy(cand_items).to(dev))
+        else:
+            user_all, item_all = model._tables()
+            dev = user_all.device
+            rep = np.repeat(users, np.diff(cand_ptr))
+            scores = ops.pair_scores(user_all, item_all, torch.from_numpy(rep).to(dev), torch.from_numpy(cand_items).to(dev))
         if device_metrics:
             return M.by_user_metrics_device(scores, cand_ptr, np.asarray(n_pos), neg_num), scores
         scores = scores.cpu().numpy()

@@ -284,24 +284,39 @@ class SCHGN(GeneralRecommender):
         self._eval_cache = cache
         return cache
 
-    @torch.no_grad()
-    def full_sort_scores(self, users: torch.Tensor, topk: int | None = None, hist=None):
-        """Scores `[n_users_in_batch, n_items]` of the given users against every item; with `topk=k` the fused
-        selection `(values [n, k], indices [n, k])` instead (the score block is never materialised)."""
-        from .. import evaluation
+    def _scorer_tables(self, users: torch.Tensor):
+        """The fused scorer's operands for `users`: their projected rows and the cached item-side tables."""
         c = self._item_side()
         e = self.emb_size
-        users = users.to(c["user_final"].device).long().reshape(-1)
         u = c["user_final"][users]
         Wk, bk = self.W_concat.weight, self.W_concat.bias               # [e, 3e]: user | item | user * item
-        return evaluation.schgn_pair_scores(
-            topk=topk, user_ids=users, hist=hist,
+        return dict(
             user_final=u, user_key=u @ c["Wi_user"], user_comp=u @ c["Wc_user"] + c["bc"],
             user_hidden=u @ Wk[:, :e].t() + bk, W_item=Wk[:, e:2 * e].contiguous(), W_prod=Wk[:, 2 * e:].contiguous(),
             w_out=self.output_mlp.weight.reshape(-1).contiguous(), h_ingre=self.h_att_ingre.weight.reshape(-1),
             h_comp=self.h_att_comp.weight.reshape(-1), codes=c["codes"], nums=c["nums"], ingre_key=c["ingre_key"],
             ingre_final=c["ingre_final"], ingre_comp=c["ingre_comp"], img_key=c["img_key"], comps=c["comps"],
             comp_keys=c["comp_keys"])
+
+    @torch.no_grad()
+    def full_sort_scores(self, users: torch.Tensor, topk: int | None = None, hist=None):
+        """Scores `[n_users_in_batch, n_items]` of the given users against every item; with `topk=k` the fused
+        selection `(values [n, k], indices [n, k])` instead (the score block is never materialised)."""
+        from .. import evaluation
+        users = users.to(self._item_side()["user_final"].device).long().reshape(-1)
+        return evaluation.schgn_pair_scores(topk=topk, user_ids=users, hist=hist, **self._scorer_tables(users))
+
+    @torch.no_grad()
+    def by_user_scores(self, users: torch.Tensor, cand_ptr, cand_items: torch.Tensor, block_pairs: int = 1 << 22):
+        """By-user evaluation scores: user `users[r]` against its candidate list `cand_items[cand_ptr[r]:cand_ptr[r+1]]`
+        (host `cand_ptr` from 0), each list scored as `inference_by_user` scores it in one batch -- including the
+        reference's `.view(b, -1)` mixing of the list's component logits, so a score depends on the list's order and
+        length.  Returns the flat fp32 device scores in list order.  Fused kernels `fr_schgn_attend_pairs` /
+        `fr_schgn_score_pairs` over the cached item-side tables (`train.mark_parameters_updated` invalidates them)."""
+        from .. import evaluation
+        users = torch.as_tensor(users).to(self._item_side()["user_final"].device).long().reshape(-1)
+        return evaluation.schgn_by_user_scores(cand_ptr, cand_items, block_pairs=block_pairs,
+                                               **self._scorer_tables(users))
 
     def full_sort_predict(self, batch_data):
         """schgn.py:318-345: the batch user(s) against all items; `[n_items]` for one user (what
