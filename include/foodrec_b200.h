@@ -132,7 +132,8 @@ int fr_spmm_csr_f32_grouped(const fr_spmm_task *tasks_host, int32_t n_tasks, int
  *   reg = (1/reg_den) * sum_g sqrt(sum over rows r in group g of |T_g[idx_g[r]]|^2)
  *
  * `emb` is the propagated table [n_rows, d] with users first and items from row `item_off`.
- * Groups: up to FR_MAX_REG_GROUPS (table pointer, int64 index pointer, count) triples; an index
+ * Groups: up to FR_MAX_REG_GROUPS (table pointer, int64 index pointer, count) triples (a group of count 0 has norm 0,
+ * no gradient, and may pass a NULL index pointer); an index
  * equal to `pad_idx[g]` (>= 0) contributes a zero row (nn.Embedding padding_idx semantics are the
  * caller's: the padding row is stored as zeros in the reference, so pad handling only matters for
  * the backward, where that row must receive no gradient).
@@ -392,8 +393,10 @@ int fr_spmm_csr_f32_push(const int32_t *seg, int64_t n_seg, const int32_t *long_
  * purpose: rows with a zero gradient still move while their first moment decays.  HealthRec's trainable raw-feature
  * tables (cikm_model.py:83,87) make this the largest HBM stream of its step.
  * Hyper-parameters are doubles like torch's python floats: `1 - beta` is formed in double and then rounded to fp32.
- *   step_dev    device int32, the number of steps taken so far (incremented by the call)
- *   scalars_dev device float[2] scratch */
+ *   step_dev    device int32, the number of steps taken so far (incremented once per call)
+ *   scalars_dev device float[2] scratch
+ * More than FR_ADAM_MAX_TENSORS non-empty tensors take several launches, each tensor exactly one; zero-size tensors
+ * are skipped.  Every tensor is validated before the first launch, so a rejected call changes nothing. */
 #define FR_ADAM_MAX_TENSORS 64
 typedef struct fr_adam_tensor {
     float *param;

@@ -102,21 +102,27 @@ extern "C" int fr_adam_step(const fr_adam_tensor *tensors_host, int32_t n_tensor
     FR_REQUIRE(n_tensors >= 0 && (n_tensors == 0 || tensors_host) && step_dev && scalars_dev, "fr_adam_step: bad argument");
     FR_REQUIRE(lr >= 0.0 && beta1 >= 0.0 && beta1 < 1.0 && beta2 >= 0.0 && beta2 < 1.0 && eps >= 0.0,
                "fr_adam_step: lr=%g betas=(%g, %g) eps=%g", lr, beta1, beta2, eps);
+    // every tensor is checked before anything is launched: a rejected call leaves the parameters, the moments and the
+    // step counter as they were
+    for (int32_t t = 0; t < n_tensors; ++t) {
+        const fr_adam_tensor &h = tensors_host[t];
+        FR_REQUIRE(h.n >= 0, "fr_adam_step: tensor %d has a negative extent", t);
+        FR_REQUIRE(h.n == 0 || (h.param && h.grad && h.exp_avg && h.exp_avg_sq), "fr_adam_step: tensor %d: null pointer", t);
+    }
     cudaStream_t st = (cudaStream_t)stream;
     {
         fr::LaunchTimer _lt("adam_prepare_kernel", st);
         adam_prepare_kernel<<<1, 1, 0, st>>>(step_dev, scalars_dev, lr, beta1, beta2);
         if (int rc = fr::check_launch("fr_adam_step/prepare")) return rc;
     }
-    for (int32_t t0 = 0; t0 < n_tensors; t0 += FR_ADAM_MAX_TENSORS) {
+    // one cursor across the launches: each non-empty tensor lands in exactly one batch of <= FR_ADAM_MAX_TENSORS
+    for (int32_t t = 0; t < n_tensors;) {
         Tensors T;
         T.count = 0;
         long long chunks = 0;
-        for (int32_t t = t0; t < n_tensors && T.count < FR_ADAM_MAX_TENSORS; ++t) {
+        for (; t < n_tensors && T.count < FR_ADAM_MAX_TENSORS; ++t) {
             const fr_adam_tensor &h = tensors_host[t];
-            FR_REQUIRE(h.n >= 0, "fr_adam_step: tensor %d has a negative extent", t);
             if (h.n == 0) continue;
-            FR_REQUIRE(h.param && h.grad && h.exp_avg && h.exp_avg_sq, "fr_adam_step: tensor %d: null pointer", t);
             const int k = T.count++;
             T.p[k] = h.param;
             T.g[k] = h.grad;

@@ -186,7 +186,8 @@ int fill_groups(Groups &g, int n_groups, const float *const *tab, const int64_t 
     g.start[0] = 0;
     for (int i = 0; i < FR_MAX_REG_GROUPS; ++i) {
         const bool on = i < n_groups;
-        FR_REQUIRE(!on || (tab[i] && idx[i] && cnt[i] >= 0), "rank_loss: bad regulariser group %d", i);
+        // an empty group (cnt 0) owns no task, so its index pointer is never read and may be NULL (an empty tensor's)
+        FR_REQUIRE(!on || (tab[i] && cnt[i] >= 0 && (idx[i] || cnt[i] == 0)), "rank_loss: bad regulariser group %d", i);
         g.tab[i] = on ? tab[i] : nullptr;
         g.idx[i] = on ? idx[i] : nullptr;
         g.dtab[i] = (on && dtab) ? dtab[i] : nullptr;

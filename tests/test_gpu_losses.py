@@ -110,32 +110,85 @@ def test_distance_correlation_golden_and_grad():
     close(y.grad, y64.grad.numpy(), rtol=1e-4)
 
 
-@pytest.mark.parametrize("n", [100, 1024])
-def test_three_view_dcor_vs_oracle(n):
+THREE = ((0, 1), (0, 2), (2, 1))
+DCOR_CASES = ([(100, 64, THREE, None), (1024, 64, THREE, None)]
+              # d = 32 instantiations; n % 4 != 0 takes the scalar Dm stores and W fetches, n < 64 a partial tile
+              + [(n, 32, THREE, None) for n in (1, 2, 3, 63, 65, 97, 2048)]
+              + [(97, 32, ((0, 1),), None),         # two views, one pair
+                 (65, 64, ((1, 0),), None),         # a reversed pair
+                 (63, 64, THREE, 1)])               # view 1 needs no gradient (its d_tab is NULL)
+
+
+def _dcor_id(case):
+    n, d, pairs, frozen = case
+    if d == 64 and pairs == THREE and frozen is None and n in (100, 1024):
+        return str(n)                                     # the original cases keep their ids
+    return f"{n}-d{d}-" + "".join(f"{a}{b}" for a, b in pairs) + ("" if frozen is None else f"-frozen{frozen}")
+
+
+@pytest.mark.parametrize("n,d,pairs,frozen", DCOR_CASES, ids=[_dcor_id(c) for c in DCOR_CASES])
+def test_three_view_dcor_vs_oracle(n, d, pairs, frozen):
     from foodrec_b200 import ops
     from oracle import losses
     torch.manual_seed(n)
     rows = 3000
-    tabs = [(torch.randn(rows + k * 10, 64) * 0.1) for k in range(3)]
+    V = 1 + max(max(ab) for ab in pairs)
+    tabs = [(torch.randn(rows + k * 10, d) * 0.1) for k in range(V)]
     idx = torch.randint(0, rows, (n,))
-    idx[5] = idx[17]  # duplicate rows in the batch (same item as pos and neg)
-    w = torch.tensor([0.3, 1.0, -0.5])
+    if n > 17:
+        idx[5] = idx[17]  # duplicate rows in the batch (same item as pos and neg)
+    w = torch.tensor([0.3, 1.0, -0.5][:len(pairs)] if len(pairs) > 1 else [-0.7])   # per-term upstream gradients
     refs = {}
     for dt in (torch.float32, torch.float64):
-        ts = [t.detach().clone().to(dt).requires_grad_(True) for t in tabs]
-        a, b, c = (t[idx] for t in ts)
-        ref = torch.stack([losses.correlation_distance(a, b), losses.correlation_distance(a, c),
-                           losses.correlation_distance(c, b)]).reshape(-1)
+        ts = [t.detach().clone().to(dt).requires_grad_(k != frozen) for k, t in enumerate(tabs)]
+        views = [t[idx] for t in ts]
+        ref = torch.stack([losses.correlation_distance(views[a], views[b]) for a, b in pairs]).reshape(-1)
         (ref * w.to(dt)).sum().backward()
-        refs[dt] = (ref.detach().numpy(), [t.grad.numpy() for t in ts])
-    tabs_d = [t.cuda().requires_grad_(True) for t in tabs]
-    out = ops.dcor_terms(tabs_d, idx.cuda(), [(0, 1), (0, 2), (2, 1)])
+        refs[dt] = (ref.detach().numpy(), [None if t.grad is None else t.grad.numpy() for t in ts])
+    tabs_d = [t.cuda().requires_grad_(k != frozen) for k, t in enumerate(tabs)]
+    out = ops.dcor_terms(tabs_d, idx.cuda(), list(pairs))
     (out * w.cuda()).sum().backward()
+    # n <= 2: two points are always perfectly distance-correlated, so each term is 1 up to the 1e-8 / 1e-10
+    # stabilisers and its float64 gradient is O(1e-8) (exactly 0 at n = 1).  Against distances of order 1 fp32 keeps
+    # none of those stabilisers (half an ulp of 1 is 6e-8), so the kernel's gradient there is the cancellation
+    # noise of a few u times the O(1) partial derivatives it sums: the floor 1e-5 sum|w| is two orders above that.
+    atol = 1e-5 * float(w.abs().sum()) if n <= 2 else 0.0
     close(out, refs[torch.float64][0], rtol=1e-5)
-    close(out, refs[torch.float32][0], rtol=1e-4)
-    for td, g64, g32 in zip(tabs_d, refs[torch.float64][1], refs[torch.float32][1]):
-        close(td.grad, g64, rtol=1e-4)
-        close(td.grad, g32, rtol=1e-2)  # the fp32 autograd reference is itself ~5e-3 noisy at n=1024 (see above)
+    original = d == 64 and pairs == THREE and frozen is None
+    if original:
+        close(out, refs[torch.float32][0], rtol=1e-4)
+    for k, (td, g64, g32) in enumerate(zip(tabs_d, refs[torch.float64][1], refs[torch.float32][1])):
+        if k == frozen:
+            assert td.grad is None
+            continue
+        close(td.grad, g64, rtol=1e-4, atol=atol)
+        if original:
+            close(td.grad, g32, rtol=1e-2)  # the fp32 autograd reference is itself ~5e-3 noisy at n=1024 (see above)
+
+
+def test_dcor_backward_into_aliased_gradient():
+    """`fr_dcor_bwd` may be handed the same gradient table for two views (the header allows aliasing): the atomics
+    then add both views' gradients into it.  Views 0 and 1 are two tables of one height sharing d_tab, view 2 has
+    its own; compared with the float64 sum of the two views' gradients."""
+    from foodrec_b200 import ops
+    from oracle import losses
+    torch.manual_seed(21)
+    n, rows = 97, 500
+    tabs = [torch.randn(rows, 32) * 0.1, torch.randn(rows, 32) * 0.1, torch.randn(rows + 9, 32) * 0.1]
+    idx = torch.randint(0, rows, (n,))
+    w = torch.tensor([0.3, 1.0, -0.5])
+    ts = [t.double().requires_grad_(True) for t in tabs]
+    views = [t[idx] for t in ts]
+    ref = torch.stack([losses.correlation_distance(views[a], views[b]) for a, b in THREE]).reshape(-1)
+    (ref * w.double()).sum().backward()
+    tabs_d = [t.cuda() for t in tabs]
+    idx_d = idx.cuda()
+    out, state = ops._dcor_forward(tabs_d, idx_d, list(THREE), 1.0)
+    close(out[:3], ref.detach().numpy(), rtol=1e-5)
+    shared, own = torch.zeros(rows, 32, device="cuda"), torch.zeros(rows + 9, 32, device="cuda")
+    ops._dcor_backward(tabs_d, idx_d, list(THREE), state, w.cuda(), [shared, shared, own])
+    close(shared, (ts[0].grad + ts[1].grad).numpy(), rtol=1e-4)
+    close(own, ts[2].grad.numpy(), rtol=1e-4)
 
 
 def test_info_nce_golden():
@@ -148,21 +201,44 @@ def test_info_nce_golden():
     close(h.grad, g["nce/gh"], rtol=1e-4)
 
 
-@pytest.mark.parametrize("rows,temperature,norm", [(1024, 0.5, True), (130, 0.2, True), (257, 0.5, False)])
-def test_info_nce_vs_oracle(rows, temperature, norm):
-    """Fused NT-Xent (one Gram matrix) vs the reference's four-block formulation restated in the oracle,
-    including an odd trailing row (ignored, zero gradient) and the un-normalised variant."""
+NCE_ORIGINAL = [(1024, 0.5, True, 64), (130, 0.2, True, 64), (257, 0.5, False, 64)]
+
+
+NCE_CASES = NCE_ORIGINAL + [
+    (1024, 0.5, True, 32), (257, 0.5, False, 32),         # the d = 32 instantiations
+    (2, 0.5, True, 64), (3, 2.0, False, 32),              # b = 1
+    (66, 0.05, True, 32), (131, 2.0, True, 64),           # b = 33, 65
+    (1400, 0.05, True, 64), (1401, 2.0, False, 32),       # b = 700
+]
+
+
+@pytest.mark.parametrize("rows,temperature,norm,d", NCE_CASES,     # the original cases keep their ids
+                         ids=["-".join(map(str, c[:3] if c in NCE_ORIGINAL else c)) for c in NCE_CASES])
+def test_info_nce_vs_oracle(rows, temperature, norm, d):
+    """Fused NT-Xent (one Gram matrix) vs the reference's four-block formulation restated in the oracle, in float64
+    (and in fp32 for the original cases), including an odd trailing row (ignored, zero gradient), the
+    un-normalised variant, small and large temperatures and an upstream gradient != 1."""
     from foodrec_b200 import ops
     from oracle import losses
     torch.manual_seed(rows)
-    h = (torch.randn(rows, 64) * (1.0 if norm else 0.3)).requires_grad_(True)
+    g = 1.7
+    h = (torch.randn(rows, d) * (1.0 if norm else 0.3)).requires_grad_(True)
     ref = losses.info_nce(h, temperature=temperature, hidden_norm=norm)
-    ref.backward()
+    (ref * g).backward()
+    h64 = h.detach().double().requires_grad_(True)
+    ref64 = losses.info_nce(h64, temperature=temperature, hidden_norm=norm)
+    (ref64 * g).backward()
     hd = h.detach().cuda().requires_grad_(True)
     out = ops.info_nce(hd, temperature=temperature, hidden_norm=norm)
-    out.backward()
-    close(out, ref.detach().numpy())
-    close(hd.grad, h.grad.numpy(), rtol=2e-5)
+    (out * g).backward()
+    # b = 1: after the mask each row's only logit is its positive, so loss and gradient are exactly 0 in exact
+    # arithmetic; a logsumexp rounded by an ulp of |G| <= 1 / temperature would leave ~1e-7, hence the floor
+    atol = 1e-6 * g if rows // 2 == 1 else 0.0
+    close(out, ref64.detach().numpy(), rtol=1e-5, atol=atol)
+    close(hd.grad, h64.grad.numpy(), rtol=1e-4, atol=atol)
+    if (rows, temperature, norm, d) in NCE_ORIGINAL:
+        close(out, ref.detach().numpy())
+        close(hd.grad, h.grad.numpy(), rtol=2e-5)
 
 
 def test_cosine_mean_vs_torch():
