@@ -388,7 +388,8 @@ int fr_spmm_csr_f32_push(const int32_t *seg, int64_t n_seg, const int32_t *long_
                          int32_t n_peers, int64_t row_off, void *stream);
 
 /* Dense Adam over many tensors in one launch (plus a one-thread prologue that advances the device-side step counter
- * and derives the bias corrections, so the pair replays inside a CUDA graph).  Replaces `optim.Adam(...).step()` of
+ * and derives the bias corrections, so the pair replays inside a CUDA graph).  `lr` is a kernel argument here, fixed
+ * at capture; fr_optim_step below reads it from the device instead.  Replaces `optim.Adam(...).step()` of
  * FoodRec/common/trainer.py:144,205 with torch.optim.Adam's arithmetic (amsgrad = False, weight_decay = 0); dense on
  * purpose: rows with a zero gradient still move while their first moment decays.  HealthRec's trainable raw-feature
  * tables (cikm_model.py:83,87) make this the largest HBM stream of its step.
@@ -407,6 +408,45 @@ typedef struct fr_adam_tensor {
 } fr_adam_tensor;
 int fr_adam_step(const fr_adam_tensor *tensors_host, int32_t n_tensors, double lr, double beta1, double beta2, double eps,
                  int32_t *step_dev, float *scalars_dev, void *stream);
+
+/* The learners of the reference trainer's optimizer factory (FoodRec/common/trainer.py:137-154: Adam, SGD, Adagrad,
+ * RMSprop with `lr` and `weight_decay`, every other option at torch's default) on the same multi-tensor launches as
+ * fr_adam_step, which runs the FR_OPTIM_ADAM rule of this entry point.  Arithmetic and its order follow torch 2.11's
+ * `_single_tensor_*` functions; with wd != 0 the gradient is first replaced by g' = g + wd p (torch's L2 term, not
+ * AdamW's decoupled decay):
+ *   FR_OPTIM_ADAM     state0 = exp_avg, state1 = exp_avg_sq, step_dev   fr_adam_step's update on g'     28 B / param
+ *   FR_OPTIM_SGD      no state (momentum 0)                             p += (-lr) g'                    12 B / param
+ *   FR_OPTIM_ADAGRAD  state0 = sum, step_dev (lr_decay 0)               s += g' g'; p += (-lr) g' / (sqrt(s) + eps)
+ *   FR_OPTIM_RMSPROP  state0 = square_avg (momentum 0, not centred)     a = a alpha + ((1 - alpha) g') g';
+ *                                                                       p += (-lr) g' / (sqrt(a) + eps)  20 B / param
+ * (Adagrad moves 20 B / param too.)  Unused state pointers of a rule may be NULL.
+ *   lr_dev      device double: the learning rate, read by the one-thread prologue of every call, so a call captured
+ *               in a CUDA graph uses the value the scalar holds at each replay.  A negative or NaN value is rejected
+ *               there: the call then changes no parameter, no state and no step, and leaves scalars_dev[0] = NaN.
+ *   step_dev    device int32, incremented once per call; required by Adam and Adagrad, may be NULL otherwise
+ *   scalars_dev device float[2] scratch
+ * Host-side rejections (unknown rule, negative eps / weight_decay, betas or alpha out of range, a NULL pointer the
+ * rule needs, a negative extent) happen before anything is launched, so they change nothing either.  Batching into
+ * launches of at most FR_ADAM_MAX_TENSORS non-empty tensors is that of fr_adam_step. */
+#define FR_OPTIM_ADAM 0
+#define FR_OPTIM_SGD 1
+#define FR_OPTIM_ADAGRAD 2
+#define FR_OPTIM_RMSPROP 3
+typedef struct fr_optim_tensor {
+    float *param;
+    const float *grad;
+    float *state0;
+    float *state1;
+    int64_t n;
+} fr_optim_tensor;
+typedef struct fr_optim_hyper {
+    double beta1, beta2;  /* Adam: betas, each in [0, 1)                   */
+    double alpha;         /* RMSprop: smoothing constant, >= 0             */
+    double eps;           /* Adam, Adagrad, RMSprop: >= 0                  */
+    double weight_decay;  /* every rule: >= 0                              */
+} fr_optim_hyper;
+int fr_optim_step(int32_t rule, const fr_optim_tensor *tensors_host, int32_t n_tensors, const fr_optim_hyper *hyper,
+                  const double *lr_dev, int32_t *step_dev, float *scalars_dev, void *stream);
 
 /* Measurement probe (not on the product path): gathers `n_idx` rows of a d = 64 table and does nothing else;
  * its bytes/s is the gather roofline the propagation kernel is compared with (scripts/microbench_gather_roofline.py).

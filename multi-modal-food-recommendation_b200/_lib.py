@@ -43,6 +43,7 @@ SIGNATURES = {
     "fr_spmm_task_blocks": (_i64, [_i64]),
     "fr_spmm_csr_f32_grouped": (C.c_int, [_p, _i32, _i32, _p, _i64, _p]),
     "fr_adam_step": (C.c_int, [_p, _i32, C.c_double, C.c_double, C.c_double, C.c_double, _p, _p, _p]),
+    "fr_optim_step": (C.c_int, [_i32, _p, _i32, _p, _p, _p, _p, _p]),
     "fr_rank_loss_ws_floats": (_i64, []),
     "fr_rank_loss_fwd": (C.c_int, [_p, _i32, _i64, _p, _p, _p, _i32, _f32, _i32, _p, _p, _p, _f32, _p, _p, _p, _p, _p]),
     "fr_rank_loss_bwd": (C.c_int, [_p, _i32, _i64, _p, _p, _p, _i32, _p, _p, _p, _i32, _p, _p, _p, _p, _f32, _p, _p, _p, _p]),
@@ -109,6 +110,20 @@ class SpmmTask(C.Structure):
 class AdamTensor(C.Structure):
     """`fr_adam_tensor` of include/foodrec_b200.h."""
     _fields_ = [("param", _p), ("grad", _p), ("exp_avg", _p), ("exp_avg_sq", _p), ("n", _i64)]
+
+
+OPTIM_ADAM, OPTIM_SGD, OPTIM_ADAGRAD, OPTIM_RMSPROP = 0, 1, 2, 3     # FR_OPTIM_* of include/foodrec_b200.h
+
+
+class OptimTensor(C.Structure):
+    """`fr_optim_tensor` of include/foodrec_b200.h."""
+    _fields_ = [("param", _p), ("grad", _p), ("state0", _p), ("state1", _p), ("n", _i64)]
+
+
+class OptimHyper(C.Structure):
+    """`fr_optim_hyper` of include/foodrec_b200.h."""
+    _fields_ = [("beta1", C.c_double), ("beta2", C.c_double), ("alpha", C.c_double), ("eps", C.c_double),
+                ("weight_decay", C.c_double)]
 
 
 for _name, (_res, _args) in SIGNATURES.items():
